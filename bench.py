@@ -3,9 +3,14 @@
 paired Rosenbrock, n = 1e7, fp64, m = 10, More-Thuente line search, x0 = 0, on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--solver-loop resident|host]
+                  [--dump-outputs DIR]
   (N > 1: launched under torchrun, one rank per GPU; c2/c3: n is sharded over the ranks ("strong" scaling);
    c5: --sharding problems (default; ranks take whole problems, no communication) or n (every problem split along n);
    c4: replicas only, N = 1)
+
+K steps are timed.  --dump-outputs DIR (one GPU) writes what the last timed step returned as DIR/<name>.npy, float64: x (c2, c3:
+downloaded after the timed region; c4 also grad and the trace of f), fx, gnorm, niter, nfev (c5: one entry per problem).  The inputs
+are fixed by the config, so two builds can be compared output for output.
 
 A "step" is one complete minimize() of the problem through the header-only C++ front on top of liblbfgs_b200.so (c2: 22 iterations /
 50 objective evaluations).  `value` = iterations per second with the start point already resident in HBM; `e2e` = the same with the
@@ -21,6 +26,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -59,6 +65,26 @@ def load_peaks():
         with open(path) as fh:
             return float(json.load(fh)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
+
+
+DUMP_SAMPLE = 1 << 21   # entries kept of a longer vector: 16 MB in float64, so a dump stays far below 64 MB
+
+
+def dump_outputs(outdir, arrays):
+    """Write each array as outdir/<name>.npy in float64.  A vector longer than DUMP_SAMPLE is replaced by its entries at DUMP_SAMPLE
+    sorted indices drawn with seed 0 from its length: the same entries in every run."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.size > DUMP_SAMPLE:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
+def result_arrays(r, *extra):
+    """What a caller of one minimize() receives, for --dump-outputs: the scalars and the named vectors of the result dict."""
+    return {k: r[k] for k in ("fx", "gnorm", "niter", "nfev") + extra}
 
 
 def load_traffic(key):
@@ -151,14 +177,16 @@ class ClockSampler(threading.Thread):
 # ---------------------------------------------------------------------------------------------------------------------
 # CPU legs (oracle/ is executed only here, in tests/ and in smoke())
 # ---------------------------------------------------------------------------------------------------------------------
-def load_oracle(native=True):
+def load_oracle():
+    """The restatement's timing build (-O3 -march=native), compiled for the host it is timed on into a temporary directory (the
+    tree may be read-only); the portable build of the tree when that compile fails."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import pyoracle as po
     try:
-        po.build(native=native)   # native build happens on the box it is timed on
-        return po, po.Oracle("orc", native=native)
+        with tempfile.TemporaryDirectory(prefix="lbfgs_b200_bench_") as tmp:
+            return po, po.Oracle("orc", path=po.build_native(tmp))   # loaded before the directory is removed
     except Exception:
-        return po, po.Oracle("orc", native=False)
+        return po, po.Oracle("orc")
 
 
 def cpu_solve(po, orc, name, sum_mode, problem=0, max_iterations=None):
@@ -184,7 +212,7 @@ def cpu_solve(po, orc, name, sum_mode, problem=0, max_iterations=None):
 def cpu_baseline_block(name, gpu_niter=None, gpu_nfev=None, gpu_fx=None):
     """The reported (not the target) CPU figure of the main arm: one full solve on ONE host thread -- the reference's Eigen level-1
     code is single-threaded and never enables OpenMP (SURVEY.md 8d)."""
-    po, orc = load_oracle(native=True)
+    po, orc = load_oracle()
     r = cpu_solve(po, orc, name, po.SUM_LANES8)
     out = {"value": r["niter"] / r["seconds"], "unit": "iters/s", "cores": 1, "kind": "port",
            "sample": "1 x minimize() of the same problem%s (%d iterations, %d evaluations, %.1f s), single thread like the reference's Eigen "
@@ -199,13 +227,13 @@ def cpu_baseline_block(name, gpu_niter=None, gpu_nfev=None, gpu_fx=None):
 def run_reference_arm(args, rank):
     """The reference's CPU implementation of the path on the host cores, pinned (VERDICT r1): the FULL solve of the config, ONE thread
     as `value` (the reference's own threading), the OpenMP restatement on all cores as an extra key; never truncated, never
-    self-calibrated.  --steps / --warmup bound the number of timed solves (at most 2: a solve of c2 takes ~12 s)."""
+    self-calibrated.  --steps is the number of timed solves (a solve of c2 takes ~12 s)."""
     if rank != 0:
         return
     name = args.config
-    po, orc = load_oracle(native=True)
+    po, orc = load_oracle()
     cpu_solve(po, orc, name, po.SUM_LANES8, max_iterations=1)          # untimed: first touch of the allocator, library load
-    nsolves = max(1, min(args.steps, 2))
+    nsolves = args.steps
     secs, iters, last = 0.0, 0, None
     for _ in range(nsolves):
         last = cpu_solve(po, orc, name, po.SUM_LANES8)
@@ -216,7 +244,9 @@ def run_reference_arm(args, rank):
     all_cores = {"value": allc["niter"] / allc["seconds"], "unit": "iters/s", "cores": orc.hw_threads(),
                  "note": "the same full solve by the OpenMP build of the restatement on all host threads (the reference has no such mode)"}
     sample = ("%d x the full minimize() of the config (%d iterations, %d evaluations each), 1 thread; warm-up = one 1-iteration solve; "
-              "restatement of the reference (oracle/liboracle_native.so, -O3 -march=native, 8-lane partial sums)" % (nsolves, last["niter"], last["nfev"]))
+              "restatement of the reference (oracle/, -O3 -march=native, 8-lane partial sums)" % (nsolves, last["niter"], last["nfev"]))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result_arrays(last, "x"))
     ref_headers = None
     if name == "c2":
         try:   # for the record: the unmodified reference headers themselves (over the minieigen stand-in), 3 iterations of the same solve
@@ -239,7 +269,7 @@ def run_reference_arm(args, rank):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-def main():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -255,12 +285,23 @@ def main():
     ap.add_argument("--sharding", default="problems", choices=["problems", "n"], help="c5 on N > 1 GPUs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-mode", action="store_true", help="timed region only (for runs under ncu; numbers are not bench values)")
-    args = ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64; a vector longer than "
+                         "%d entries as a fixed, seeded sample of that many)" % DUMP_SAMPLE)
+    args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
+    return args
 
+
+def main():
+    args = parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        sys.exit("--dump-outputs runs on one GPU")
 
     if args.impl == "reference":
         run_reference_arm(args, rank)
@@ -331,6 +372,7 @@ def main():
 
     line = {"metric": "lbfgs_iterations_per_sec", "unit": "iters/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
             "higher_is_better": True, "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": workload_config(name)}
+    outputs = None   # --dump-outputs: name -> array of the last timed step
 
     def device_timed(fn, steps):
         """fn() `steps` times between a barrier + synchronize on both sides; CUDA-event time on the library's stream, max over ranks."""
@@ -390,6 +432,8 @@ def main():
                 profs.append(sess.profile())
             return rr
         outs, dev_seconds = device_timed(one, args.steps)
+        if args.dump_outputs:   # before the end-to-end solves below overwrite x
+            outputs = dict(result_arrays(outs[-1]), x=sess.download())
         iters = sum(o["niter"] for o in outs)
         launches = sum(o["launches"] for o in outs)
         # ---- end to end: pinned host -> device every step, result back to the host ----
@@ -467,6 +511,7 @@ def main():
             secs += r["seconds"]; e2e_secs += r["seconds_e2e"]; iters += r["niter"]; launches += r["launches"]
         barrier()
         clocks = sampler.summary()
+        outputs = result_arrays(r, "x", "grad", "trace")
         # algorithmic bytes of one L-BFGS-B iteration at c pairs (DESIGN.md section 9): line-search trials 4n each, breakpoints + classes 5n,
         # W'd and the Cauchy build ~(2c+4)n, subspace minimisation >= (4c+8)n per BOXCQP sweep: reported as a lower bound with T trials
         nfev = r["nfev"]
@@ -503,7 +548,6 @@ def main():
             X0 = np.stack([np.random.default_rng(1000 + b).uniform(-1, 1, n_global) for b in mine])
         prm = lb.LBFGSParam(m=m_hist)
         bs = lb.BatchSession(lb.OBJ_ROSENBROCK_PAIRED, X0, prm, cfg["ls"], device=local_rank)
-        steps = max(1, min(args.steps, 3))
         for _ in range(max(1, min(args.warmup, 2))):
             res, _, _ = bs.solve(return_x=False)
         sampler.start()
@@ -515,7 +559,7 @@ def main():
             if pr:
                 profs.append(pr)
             return rr
-        outs, dev_seconds = device_timed(one_batch, steps)
+        outs, dev_seconds = device_timed(one_batch, args.steps)
         iters_rank = sum(sum(p["niter"] for p in o) for o in outs)
         iters = iters_rank if shard_n else sum_over_ranks(iters_rank)
         barrier()
@@ -526,12 +570,13 @@ def main():
         e2e_seconds = max_over_ranks(time.perf_counter() - t0)
         e2e_iters = sum(p["niter"] for p in resx) if shard_n else sum_over_ranks(sum(p["niter"] for p in resx))
         clocks = sampler.summary()
+        outputs = {k: [p[k] for p in outs[-1]] for k in ("fx", "gnorm", "niter", "nfev")}
         its = [p["niter"] for p in outs[-1]]
         rounds = [p["rounds"] for p in outs[-1]]
-        line.update({"value": iters / dev_seconds, "ms_per_step": 1e3 * dev_seconds / steps, "steps": steps, "scaling": "strong", "clocks": clocks,
+        line.update({"value": iters / dev_seconds, "ms_per_step": 1e3 * dev_seconds / args.steps, "scaling": "strong", "clocks": clocks,
                      "e2e": {"value": e2e_iters / e2e_seconds, "unit": "iters/s", "h2d_bytes_per_step": int(h2d_bytes), "d2h_bytes_per_step": int(X.nbytes),
                              "note": "one batched solve with its start points uploaded from and its solutions copied back to host memory (bytes per rank)"},
-                     "gpu_launches": steps, "launches_per_solve": 1,
+                     "gpu_launches": args.steps, "launches_per_solve": 1,
                      "solver_loop": "device-resident: ONE persistent kernel launch for the rank's whole batch",
                      "setup": {"problems_per_rank": len(mine), "n_per_gpu": n_local,
                                "sharding": "single GPU" if world == 1 else ("n of every problem split over %d ranks: one exchange per round carrying the "
@@ -547,6 +592,8 @@ def main():
         bs.close()
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

@@ -543,6 +543,15 @@ class Session:
         p = self.drv.lbfgsb200_drv_session_result(self.h)
         return np.ctypeslib.as_array(p, shape=(self.n,)).copy()
 
+    def download(self):
+        """x as the last solve() left it on the device (also when that solve did not copy it to the host)."""
+        x = np.empty(self.n)
+        err = C.create_string_buffer(256)
+        self.drv.lbfgsb200_drv_session_download.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.c_char_p, C.c_int]
+        if self.drv.lbfgsb200_drv_session_download(self.h, x.ctypes.data_as(C.POINTER(C.c_double)), err, 256):
+            raise RuntimeError("session download failed: " + err.value.decode())
+        return x
+
     def close(self):
         if self.h:
             self.drv.lbfgsb200_drv_session_destroy(self.h)

@@ -422,6 +422,21 @@ int lbfgsb200_drv_session_solve(void* handle, int from_host, int to_host, drv_re
 
 const double* lbfgsb200_drv_session_result(void* handle) { return static_cast<Session*>(handle)->pinned_out; }
 
+// The x the last solve left on the device -> x_host (n doubles), for a solve that ran with to_host = 0; synchronises.
+int lbfgsb200_drv_session_download(void* handle, double* x_host, char* err, int errlen)
+{
+    try
+    {
+        static_cast<Session*>(handle)->x.copy_to_host(x_host);
+        return 0;
+    }
+    catch (const std::exception& e)
+    {
+        if (err && errlen > 0) { std::strncpy(err, e.what(), size_t(errlen) - 1); err[errlen - 1] = 0; }
+        return -1;
+    }
+}
+
 // accounting of the session's last device-resident solve (lbfgs_b200_solver_profile; sync_ms has 3 slots); returns 1 when the
 // session runs the host-driven loop
 int lbfgsb200_drv_session_profile(void* handle, double* kernel_ms, double* ms_by_op10, unsigned long long* rounds_by_op10, double* alg_bytes_by_op10,

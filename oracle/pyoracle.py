@@ -33,10 +33,17 @@ class Result(C.Structure):
                 ("fx", C.c_double), ("gnorm", C.c_double), ("trace_len", C.c_long), ("seconds", C.c_double)]
 
 
-def build(native=False):
+def build():
     """(Re)build the checkers with oracle/Makefile.  Building the checker is not using it."""
-    targets = ["all"] + (["native"] if native else [])
-    subprocess.run(["make", "-s", "-C", HERE] + targets, check=True)
+    subprocess.run(["make", "-s", "-C", HERE, "all"], check=True)
+
+
+def build_native(outdir):
+    """The timing build of the restatement (`make native`: -O3 -march=native for the host it runs on) into outdir, so that a
+    read-only tree works; returns its path for Oracle("orc", path=...)."""
+    path = os.path.join(outdir, "liboracle_native.so")
+    subprocess.run(["make", "-s", "-C", HERE, "native", "NATIVE_LIB=" + path], check=True)
+    return path
 
 
 def _ptr(a, ctype):
@@ -44,13 +51,11 @@ def _ptr(a, ctype):
 
 
 class Oracle:
-    def __init__(self, which="orc", native=False):
+    def __init__(self, which="orc", path=None):
         assert which in ("orc", "ref")
         self.prefix = which + "_"
-        if which == "ref":
-            path = os.path.join(HERE, "_ref", "libref_lbfgspp.so")
-        else:
-            path = os.path.join(HERE, "liboracle_native.so" if native else "liboracle.so")
+        if path is None:
+            path = os.path.join(HERE, "_ref", "libref_lbfgspp.so") if which == "ref" else os.path.join(HERE, "liboracle.so")
         if not os.path.exists(path):
             raise FileNotFoundError(path)
         self.path = path

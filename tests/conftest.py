@@ -11,7 +11,7 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
 
 def pytest_configure(config):
-    config.addinivalue_line("markers", "gpu: needs a real B200 (run by the driver at round end with -m gpu)")
+    config.addinivalue_line("markers", "gpu: needs a real B200")
 
 
 @pytest.fixture(scope="session")
@@ -21,19 +21,6 @@ def orc():
     if not os.path.exists(os.path.join(ROOT, "oracle", "liboracle.so")):
         pyoracle.build()
     return pyoracle.Oracle("orc")
-
-
-@pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference headers over minieigen; exists only where /root/reference was present at build time."""
-    import pyoracle
-    path = os.path.join(ROOT, "oracle", "_ref", "libref_lbfgspp.so")
-    if not os.path.exists(path):
-        if os.path.isdir("/root/reference/include"):
-            pyoracle.build()
-        else:
-            pytest.skip("oracle/_ref not built (no /root/reference on this machine)")
-    return pyoracle.Oracle("ref")
 
 
 @pytest.fixture(scope="session")

@@ -84,3 +84,33 @@ def test_peak_lookup(bench):
         assert peak == float(json.load(open(path))["hbm_gbs"]) and src.startswith("measured")
     else:
         assert peak == 6650.0 and src.startswith("fallback")
+
+
+def test_dump_outputs_writes_float64_and_a_fixed_sample(bench, tmp_path):
+    import numpy as np
+    x = np.arange(bench.DUMP_SAMPLE + 1000, dtype=np.float64)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"x": x, "fx": 1.5, "niter": [22, 23]})
+    a = np.load(tmp_path / "a" / "x.npy")
+    assert a.dtype == np.float64 and a.size == bench.DUMP_SAMPLE and np.all(np.diff(a) > 0)   # distinct entries of x, in order
+    assert np.array_equal(a, np.load(tmp_path / "b" / "x.npy"))
+    assert np.load(tmp_path / "a" / "fx.npy") == 1.5 and np.load(tmp_path / "a" / "niter.npy").tolist() == [22.0, 23.0]
+    small = np.arange(10.0)
+    bench.dump_outputs(str(tmp_path / "c"), {"x": small})
+    assert np.array_equal(np.load(tmp_path / "c" / "x.npy"), small)
+
+
+def test_parse_args_steps_and_dump_outputs(bench):
+    assert bench.parse_args(["--steps", "7"]).steps == 7
+    assert bench.parse_args(["--dump-outputs", "out"]).dump_outputs == "out"
+    with pytest.raises(SystemExit):
+        bench.parse_args(["--steps", "0"])
+
+
+def test_cpu_leg_builds_its_checker_outside_the_tree(bench):
+    """The timing build of the checker goes to a temporary directory: bench.py writes nothing into the tree."""
+    before = sorted(os.listdir(os.path.join(ROOT, "oracle")))
+    po, orc = bench.load_oracle()
+    assert not orc.path.startswith(ROOT + os.sep) and not os.path.exists(orc.path)
+    assert sorted(os.listdir(os.path.join(ROOT, "oracle"))) == before
+    assert orc.lbfgs(po.OBJ_ROSENBROCK_PAIRED, [0.0] * 10, po.LS_MORE_THUENTE, orc.default_param())["niter"] == 21

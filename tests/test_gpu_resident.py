@@ -152,3 +152,19 @@ def test_resident_large_history(orc, m, iters):
     h = lb.LBFGSSolver(prm, "Bracketing", resident=False).minimize(lb.OBJ_QUAD_TRIDIAG, np.zeros(n), data0=d, data1=b)
     assert (h["niter"], h["nfev"]) == (g["niter"], g["nfev"]) and abs(h["fx"] - g["fx"]) <= 1e-9 * abs(g["fx"])
 
+
+@pytest.mark.parametrize("resident_loop", [True, False])
+def test_session_download_returns_the_last_solve(resident_loop):
+    """Session.download() after a solve that left x on the device gives the x that the same solve copies back with to_host=True."""
+    n = 4098
+    prm = lb.LBFGSParam(m=10)
+    sess = lb.Session(lb.OBJ_ROSENBROCK_PAIRED, np.zeros(n), prm, "MoreThuente", resident=resident_loop)
+    r = sess.solve()
+    x = sess.download()
+    r2 = sess.solve(to_host=True)
+    x2 = sess.result()
+    sess.close()
+    lone = lb.LBFGSSolver(prm, "MoreThuente", resident=resident_loop).minimize(lb.OBJ_ROSENBROCK_PAIRED, np.zeros(n))
+    assert (r["niter"], r["nfev"], r["fx"]) == (r2["niter"], r2["nfev"], r2["fx"])
+    assert np.array_equal(x, x2)
+    assert (r["niter"], r["nfev"]) == (lone["niter"], lone["nfev"]) and np.max(np.abs(x - lone["x"])) <= 1e-8

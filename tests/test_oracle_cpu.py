@@ -1,10 +1,10 @@
-"""CPU tests of the checker itself: the restatement must reproduce (a) the unmodified reference headers run over
-minieigen, bit for bit, wherever that build exists, and (b) the golden vectors frozen from that build, everywhere."""
+"""CPU tests of the checker itself: the restatement must reproduce the unmodified reference headers run over minieigen, bit
+for bit, on the inputs whose results were frozen from that build (golden/lbfgs_ref.json, golden/pins_ref.json)."""
 import numpy as np
 import pytest
 
 import pyoracle as po
-from util import LS, golden_cases, same_run, unhex
+from util import LS, fingerprint, golden_cases, golden_pins, pin_cases, unhex
 
 
 def run_golden_lbfgs(orc, c):
@@ -90,77 +90,36 @@ def test_gram_form_matches_two_loop_on_cpu(orc):
         assert abs(a["fx"] - b["fx"]) <= 1e-10 * max(1.0, abs(a["fx"]))
 
 
-# ---- against the unmodified reference headers (only where oracle/_ref could be built) ------------------------------
-def test_pin_against_reference_headers(orc, ref):
-    rng = np.random.default_rng(1)
-    for n in (2, 6, 24, 100, 2002):
-        for t in range(6):
-            x0 = rng.uniform(-1, 1, n)
-            for ls in range(4):
-                p = ref.default_param(max_linesearch=256, m=3 + t % 8)
-                assert same_run(ref.lbfgs(po.OBJ_ROSENBROCK_PAIRED, x0, ls, p), orc.lbfgs(po.OBJ_ROSENBROCK_PAIRED, x0, ls, p))
-    d, b, _ = po.quad_tridiag_data(3000)
-    for ls in range(4):
-        p = ref.default_param(m=20)
-        assert same_run(ref.lbfgs(po.OBJ_QUAD_TRIDIAG, np.zeros(3000), ls, p, data0=d, data1=b),
-                        orc.lbfgs(po.OBJ_QUAD_TRIDIAG, np.zeros(3000), ls, p, data0=d, data1=b))
+# ---- against the unmodified reference headers: their results on these inputs, frozen in golden/pins_ref.json ------------------
+def check_pins(orc, group):
+    frozen = golden_pins(group)
+    cases = pin_cases(group)
+    assert sorted(name for name, _ in cases) == sorted(frozen)
+    for name, run in cases:
+        assert fingerprint(run(orc)) == frozen[name], name
 
 
-def test_pin_float32_against_reference_headers(orc, ref):
-    for ls in range(4):
-        p = ref.default_param()
-        a = ref.lbfgs(po.OBJ_ROSENBROCK_PAIRED, np.zeros(10), ls, p, dtype=np.float32)
-        b = orc.lbfgs(po.OBJ_ROSENBROCK_PAIRED, np.zeros(10), ls, p, dtype=np.float32)
-        assert same_run(a, b)
+def test_pin_against_reference_headers(orc):
+    check_pins(orc, "lbfgs")
 
 
-def test_pin_apply_Hv_against_reference_headers(orc, ref):
-    rng = np.random.default_rng(3)
-    n, m = 1000, 5
-    for npairs in (0, 1, 4, 5, 6, 13):
-        S = rng.standard_normal((npairs, n))
-        Y = S + 0.1 * rng.standard_normal((npairs, n))
-        v = rng.standard_normal(n)
-        ra, _, ta = ref.apply_Hv(S, Y, v, -1.0, m)
-        rb, _, tb = orc.apply_Hv(S, Y, v, -1.0, m)
-        assert np.array_equal(ra, rb) and ta == tb
+def test_pin_float32_against_reference_headers(orc):
+    check_pins(orc, "lbfgs_f32")
 
 
-def test_pin_lbfgsb_against_reference_headers(orc, ref):
+def test_pin_apply_Hv_against_reference_headers(orc):
+    check_pins(orc, "apply_Hv")
+
+
+def test_pin_lbfgsb_against_reference_headers(orc):
     """Cauchy point, subspace minimisation, Bunch-Kaufman LDL' and the L-BFGS-B driver, bit for bit: mixed finite /
     infinite / degenerate (l == u) bounds, history sizes 1..10, 0..10 BOXCQP sweeps, delta-based stopping."""
-    rng = np.random.default_rng(3)
-    for obj in (po.OBJ_ROSENBROCK_CHAINED, po.OBJ_ROSENBROCK_PAIRED, po.OBJ_QUAD_SHIFT, po.OBJ_QUAD_TRIDIAG):
-        for n in (2, 4, 10, 25, 26, 100):
-            if obj == po.OBJ_ROSENBROCK_PAIRED and n % 2:
-                continue
-            for trial in range(6):
-                lo = rng.uniform(-2, 1, n)
-                hi = lo + rng.uniform(0, 3, n)
-                if trial == 0:
-                    lo[:], hi[:] = 2.0, 4.0
-                elif trial == 1:
-                    lo[:], hi[:] = -np.inf, np.inf
-                elif trial == 2:
-                    hi[::3] = lo[::3]
-                elif trial == 3:
-                    lo[::2], hi[1::3] = -np.inf, np.inf
-                x0 = rng.uniform(-3, 5, n)
-                d0, d1 = po.quad_tridiag_data(n, seed=trial)[:2] if obj == po.OBJ_QUAD_TRIDIAG else (None, None)
-                kw = dict(m=int(rng.choice([1, 2, 3, 6, 10])), max_iterations=int(rng.choice([0, 5, 50])),
-                          max_submin=int(rng.choice([0, 1, 10])), past=int(rng.choice([0, 0, 2])))
-                if kw["past"]:
-                    kw["delta"] = 1e-8
-                a = orc.lbfgsb(obj, x0, lo, hi, orc.default_param(lbfgsb=True, **kw), data0=d0, data1=d1)
-                b = ref.lbfgsb(obj, x0, lo, hi, ref.default_param(lbfgsb=True, **kw), data0=d0, data1=d1)
-                assert same_run(a, b), (obj, n, trial, kw)
+    check_pins(orc, "lbfgsb")
 
 
-def test_pin_lbfgsb_larger_against_reference_headers(orc, ref):
-    for n, obj in ((2000, po.OBJ_ROSENBROCK_CHAINED), (5000, po.OBJ_ROSENBROCK_PAIRED)):
-        a = orc.lbfgsb(obj, np.full(n, 3.0), 2.0, 4.0, orc.default_param(lbfgsb=True))
-        b = ref.lbfgsb(obj, np.full(n, 3.0), 2.0, 4.0, ref.default_param(lbfgsb=True))
-        assert same_run(a, b) and a["status"] == "ok"
+def test_pin_lbfgsb_larger_against_reference_headers(orc):
+    check_pins(orc, "lbfgsb_larger")
+    assert all(c["status"] == "ok" for c in golden_pins("lbfgsb_larger").values())
 
 
 def test_lbfgsb_parameter_and_bound_errors(orc):
