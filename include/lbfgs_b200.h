@@ -295,7 +295,11 @@ const void* lbfgs_b200_solver_final_grad(const lbfgs_b200_solver* s);   /* devic
 const void* lbfgs_b200_solver_final_grad_of(const lbfgs_b200_solver* s, int problem);
 lbfgs_b200_hist* lbfgs_b200_solver_history(lbfgs_b200_solver* s);       /* the S/Y ring of problem 0 as left by the last solve   */
 lbfgs_b200_hist* lbfgs_b200_solver_history_of(lbfgs_b200_solver* s, int problem);
-/* x_inout: device vector (start point in, solution out).  trace_host (optional): f of every evaluation. */
+/* x_inout: device vector (start point in, solution out).  trace_host (optional): f of every evaluation.
+ * data0/data1 (the tridiagonal quadratic's d and b): device vectors, 16-byte aligned.  They are read by bulk copies of whole 256-byte
+ * lines, so each must stay readable up to n rounded up to a multiple of 256 bytes (32 fp64 / 64 fp32 elements); the values past n
+ * are never used.  Memory from lbfgs_b200_malloc(n * elem_bytes) satisfies both.  A misaligned pointer fails with
+ * LBFGS_B200_ERR_INVALID, as does a configuration whose passes do not fit the kernel's staging ring (LBFGS_B200_STAGES). */
 lbfgs_b200_status lbfgs_b200_solver_minimize_f64(lbfgs_b200_solver* s, int objective, const double* data0, const double* data1,
                                                  const lbfgs_b200_param* prm, int line_search, double* x_inout,
                                                  double* trace_host, long long trace_cap, lbfgs_b200_outcome* out);
@@ -303,7 +307,9 @@ lbfgs_b200_status lbfgs_b200_solver_minimize_f32(lbfgs_b200_solver* s, int objec
                                                  const lbfgs_b200_param* prm, int line_search, float* x_inout,
                                                  double* trace_host, long long trace_cap, lbfgs_b200_outcome* out);
 /* Batch: problem b starts from x_inout + b*ldx (device) and leaves its solution there; data0/data1 (optional) per problem at
- * data + b*ldd (ldd = 0: shared by all problems); outs[batch]. */
+ * data + b*ldd (ldd = 0: shared by all problems; otherwise ldd >= n and ldd * elem_bytes a multiple of 16, else
+ * LBFGS_B200_ERR_INVALID).  The padded tail above applies to every problem's vectors: a buffer of (batch - 1) * ldd elements plus n
+ * rounded up to 256 bytes is enough.  outs[batch]. */
 lbfgs_b200_status lbfgs_b200_solver_minimize_batch_f64(lbfgs_b200_solver* s, int objective, const double* data0, const double* data1,
                                                        int64_t ldd, const lbfgs_b200_param* prm, int line_search, double* x_inout,
                                                        int64_t ldx, lbfgs_b200_outcome* outs);

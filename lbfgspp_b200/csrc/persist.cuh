@@ -34,14 +34,14 @@
 #pragma once
 
 #include "../../include/LBFGSpp/LineSearchCore.h"
+#include "persist_geometry.h"
 
 namespace lb {
 
 constexpr int kMaxPast = 64;
 constexpr int kPThreads = kGramMaxThreads;   // 768: one CTA per SM
 constexpr int kPWarps = kPThreads / 32;
-constexpr int kPStageBytes = kGramStages * 4 * kGramTE * 8;   // dynamic shared memory of the kernel: 196608 bytes
-constexpr int kPMaxStages = 4;
+static_assert(kPStageBytes == kGramStages * 4 * kGramTE * 8, "the staging ring is the Gram kernels' three stages of four fp64 tiles");
 constexpr int kPCache = 4;                   // problems whose leader-side state is kept in shared memory
 
 enum { POP_IDLE = 0, POP_FIRST = 1, POP_TRIAL = 2, POP_DOTS_FORM = 3, POP_DOTS_PLAIN = 4, POP_COMBINE = 5, POP_COMBINE_TRIAL = 6, POP_RESTORE = 7,
@@ -346,7 +346,6 @@ __device__ __forceinline__ void p_trial(const OBJ& obj, const Own& own, const T*
 // shared memory by bulk copies, every tile with one 16-byte granule of margin on either side, so that x_{i-1} and x_{i+1} of a pack
 // come from the tile instead of from single-word L2 loads per pack (3x faster on config 3).  Only the two ends of the GLOBAL vector
 // take their neighbours from the halo record (n-sharding) or as 0.
-constexpr int kTrialTE = 2016;    // 63 x 32 elements: with the margins, six fp64 (xp, d) stages fit the ring
 
 template <class T, class OBJ, int MODE>
 __device__ __forceinline__ void p_trial_halo(const OBJ& obj, const Own& own, const T* __restrict__ xp, const T* __restrict__ d, T step,
@@ -358,8 +357,8 @@ __device__ __forceinline__ void p_trial_halo(const OBJ& obj, const Own& own, con
     constexpr int NVEC = NIN + DV;
     constexpr int PAD = 16 / (int)sizeof(T);                         // margin in elements = one 16-byte granule
     constexpr int TS = kTrialTE + 2 * PAD;                           // staged elements per vector per tile
-    constexpr int STAGES_MAX = kPStageBytes / (NVEC * TS * (int)sizeof(T));
-    constexpr int STAGES = STAGES_MAX > kPMaxStages ? kPMaxStages : STAGES_MAX;
+    constexpr int STAGES = trial_halo_stages((int)sizeof(T), NIN, DV);   // (kTrialTE: with the margins, six fp64 (xp, d) tiles fit the ring)
+    static_assert(STAGES >= 1, "a trial tile must fit the staging ring");
     const int tid = threadIdx.x, lane = tid & 31;
     uint64_t* full_bar = sh.full_bar;
     const T* in0 = (MODE == 1) ? xp : x;
@@ -550,8 +549,7 @@ __device__ __forceinline__ void p_dots(const PDots<T>& a, const Own& own, T* til
     const int upp = (TE / EPT) / a.split;                        // units of a tile per warp of a column group
     const SlotRuns runs(a.end, a.cnt_old, a.h.M);
     const int nrows = NRHS + 2 * a.cnt_old;
-    int stages = (int)((size_t)kPStageBytes / ((size_t)nrows * TE * sizeof(T)));
-    stages = stages > kPMaxStages ? kPMaxStages : stages;
+    const int stages = dots_stages((int)sizeof(T), TE, FORM, a.cnt_old);   // >= 1: checked by the host before the launch
     const int64_t ntl = own.ntiles(TE);
     uint64_t* full_bar = sh.full_bar;
 
@@ -690,8 +688,7 @@ __device__ __forceinline__ void p_combine(const OBJ& obj, const Own& own, const 
     const SlotRuns runs(end, c, h.M);
     const int nrows = NRHS + 2 * c;
     const size_t stage_elems = (size_t)nrows * TE + (HALO ? 2 * PAD : 0);
-    int stages = (int)((size_t)kPStageBytes / (stage_elems * sizeof(T)));
-    stages = stages > kPMaxStages ? kPMaxStages : stages;
+    const int stages = combine_stages((int)sizeof(T), TE, c, FUSE, HALO, DV);   // >= 1: checked by the host before the launch
     const int64_t n = own.n;
     const int64_t ntl = own.ntiles(TE);
     const T* s_coef = reinterpret_cast<const T*>(sh.coef);

@@ -70,6 +70,10 @@ static lbfgs_b200_status solver_minimize(lbfgs_b200_solver* s, int objective, co
     const bool coupled = objective == LBFGS_B200_OBJ_ROSENBROCK_CHAINED || objective == LBFGS_B200_OBJ_QUAD_TRIDIAG;
     if (objective == LBFGS_B200_OBJ_ROSENBROCK_PAIRED) REQUIRE(ctx, s->n % 2 == 0, "paired Rosenbrock needs an even n");
     if (objective == LBFGS_B200_OBJ_QUAD_TRIDIAG) REQUIRE(ctx, data0 && data1, "quad_tridiag needs data0 = diag, data1 = rhs");
+    // the data vectors are read by 16-byte bulk copies, from data + b*ldd on for problem b (lbfgs_b200.h)
+    REQUIRE(ctx, (uintptr_t)data0 % 16 == 0 && (uintptr_t)data1 % 16 == 0, "solver_minimize: data0 / data1 must be 16-byte aligned");
+    REQUIRE(ctx, ldd == 0 || (ldd >= s->n && (ldd * (int64_t)sizeof(T)) % 16 == 0),
+            "solver_minimize: the batch stride of the data vectors must be 0 (shared) or >= n and a multiple of 16 bytes (got %lld)", (long long)ldd);
     int64_t n_global = s->n, index_offset = ctx->index_offset;
     if (ctx->nranks > 1 && coupled)
     {
@@ -80,6 +84,13 @@ static lbfgs_b200_status solver_minimize(lbfgs_b200_solver* s, int objective, co
     }
     else if (coupled) index_offset = 0;
     if (ctx->x_active) REQUIRE(ctx, (size_t)B * (s->pstride + 4) <= (size_t)kXMaxVals, "batch of %d problems with m = %d exceeds the exchange buffer", B, s->m);
+    {
+        // every staged pass must fit at least one tile into the staging ring, or it would wait for a copy that was never issued
+        const int data_vectors = objective == LBFGS_B200_OBJ_QUAD_TRIDIAG ? 2 : 0;
+        const int stages = persist_min_stages(s->m, s->elem, 1 << s->bt_log, coupled, data_vectors);
+        REQUIRE(ctx, stages >= 1, "solver_minimize: with history blocks of %d elements (LBFGS_B200_STAGES) a pass of m = %d does not fit the staging ring",
+                1 << s->bt_log, s->m);
+    }
     const int rounds = (s->m + kGramMaxWarps - 1) / kGramMaxWarps;   // column pairs per round of the dots pass: at most one per warp
     void* kernel = persist_kernel_for<T>(objective, rounds);
     if (!kernel) return fail(ctx, LBFGS_B200_ERR_INVALID, "unknown objective id %d", objective);
@@ -264,9 +275,9 @@ lbfgs_b200_status lbfgs_b200_solver_create_batch(lbfgs_b200_ctx* ctx, int64_t n,
     s->M = m + 1;
     // block length of the tiled history: the largest power of two for which two stages of 2m+4 rows fit the kernel's staging ring
     {
-        int bt = 1024, want_stages = 2;
+        int want_stages = 2;
         if (const char* e = getenv("LBFGS_B200_STAGES")) { const int v = atoi(e); if (v >= 1 && v <= lb::kPMaxStages) want_stages = v; }
-        while (bt > 32 && (size_t)want_stages * (2 * m + 4) * bt * elem_bytes > (size_t)lb::kPStageBytes) bt >>= 1;
+        const int bt = lb::persist_block_len(m, elem_bytes, want_stages);
         s->bt_log = 0;
         while ((1 << s->bt_log) < bt) s->bt_log++;
     }
